@@ -7,6 +7,7 @@ model_dim 4096, hidden 14336, 16 x 512 = 8192 tokens per GPU, capacity_factor 1.
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29500 \
         bench.py --gpus 8 --steps 20 --warmup 5
+    python bench.py --gpus 1 --steps 20 --warmup 5 --dump-outputs /tmp/out   # + the last step's results as .npy files
     python bench.py --impl reference ...      # the UNMODIFIED reference from baseline/_ref, same metric / config
 
 Prints one JSON line on rank 0.
@@ -40,7 +41,34 @@ def parse():
     ap.add_argument('--fp8', action='store_true')                  # ours only: e4m3 forward + data-gradient GEMMs
     ap.add_argument('--graph', default='auto', choices=['auto', 'off'])     # ours, 1 GPU: replay the whole step as one CUDA graph
     ap.add_argument('--fp8_mode', default='row', choices=['row', 'mx'])   # row scales (fused engine) or MX 32-element block scales
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last step computed (loss, input gradient, parameter '
+                         'gradients and updated parameters) as DIR/<name>.npy, for output-for-output comparison of builds')
     return ap.parse_args()
+
+
+DUMP_SAMPLE = 1 << 18      # elements kept of a larger array: every dump stays far below 64 MB
+
+
+def dump_outputs(out_dir, loss, x, model):
+    """Write the loss, the input gradient and every parameter's gradient and updated value as float32 (float64 for
+    float64 tensors) .npy files.  An array of more than DUMP_SAMPLE elements is stored as a 1-D sample at fixed, seeded
+    flat indices (the same for every run of the same shapes)."""
+    import numpy as np
+    import torch
+    arrays = [('loss', loss), ('input_grad', x.grad)]
+    for name, p in model.named_parameters():
+        arrays += [('param.' + name, p), ('grad.' + name, p.grad)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays:
+        if t is None:
+            continue
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        t = t.to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu()
+        np.save(os.path.join(out_dir, name + '.npy'), t.numpy())
 
 
 def main():
@@ -174,6 +202,8 @@ def main():
             torch.cuda.synchronize()
     # Keep warming (untimed) until the step time has converged: blocks of 4 steps, stop when two consecutive blocks agree
     # within 2 % on every rank (clocks, the power-cap controller and the allocator settle within a few dozen steps).
+    # With --dump-outputs all 12 blocks run: every SGD step moves the weights, so the dumped step must be the same step
+    # of the training run each time.
     prev_blk, warm_trace = None, []
     for _ in range(12):
         w0, w1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -185,7 +215,7 @@ def main():
         warm_done += 4
         blk = maxreduce(w0.elapsed_time(w1) / 4)
         warm_trace.append(round(blk, 3))
-        if prev_blk is not None and abs(blk - prev_blk) <= 0.02 * prev_blk:
+        if args.dump_outputs is None and prev_blk is not None and abs(blk - prev_blk) <= 0.02 * prev_blk:
             break
         prev_blk = blk
     if args.impl == 'ours':
@@ -203,6 +233,7 @@ def main():
     sync()
     t_wall1 = time.time()
     gc.enable()
+    last_loss, last_x = loss, x_dev
     ms = maxreduce(e0.elapsed_time(e1))
     launches = (backend.launch_count() - launches0) if args.impl == 'ours' else None
     clocks = None
@@ -268,11 +299,17 @@ def main():
         sync()
         gc.enable()
         ms_e2e = maxreduce(f0.elapsed_time(f1))
+        # the last step's loss as the host received it; a graph replay computes the gradient of its static input x_dev
+        last_loss = loss_host[(args.steps - 1) % 2]
+        last_x = x_dev if graph_info['cuda_graph'] else slots[(args.steps - 1) % 2][0]
         e2e = {'value': world * BATCH * TOKENS * args.steps / (ms_e2e * 1e-3), 'unit': 'tokens/s',
                'h2d_bytes_per_step': x_host.numel() * x_host.element_size() + y_host.numel() * y_host.element_size(),
                'd2h_bytes_per_step': loss_host[0].numel() * loss_host[0].element_size(), 'ms_per_step': ms_e2e / args.steps, 'last_loss': last,
                'loss_read': 'asynchronous D2H copy into pinned memory behind every step, consumed by the host one step later (same in both arms)',
                'input_pipeline': 'double-buffered H2D prefetch on a copy stream (same in both arms)'}
+
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last_loss, last_x, model)
 
     tokens = world * BATCH * TOKENS * args.steps
     value = tokens / (ms * 1e-3)

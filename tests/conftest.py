@@ -28,16 +28,8 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope='session')
 def golden():
-    """Reference golden loss curves (tests/test_baseline.json of the reference; numbers only, read at test time)."""
+    """Golden loss curves of the original Tutel helloworld (the first 12 losses of each curve in its
+    tests/test_baseline.json), stored in tests/golden/losses.json."""
     import json
-    path = '/root/reference/tests/test_baseline.json'
-    local = os.path.join(ROOT, 'tests', 'golden_losses.json')
-    if os.path.exists(local):
-        with open(local) as f:
-            return json.load(f)
-    if os.path.exists(path):
-        with open(path) as f:
-            data = json.load(f)
-        return [{'top': d['top'], 'dtype': d['dtype'], 'num_local_experts': d['num_local_experts'],
-                 'losses': [float(v) for v in d['losses'][:12]]} for d in data]
-    pytest.skip('golden losses unavailable')
+    with open(os.path.join(ROOT, 'tests', 'golden', 'losses.json')) as f:
+        return json.load(f)
