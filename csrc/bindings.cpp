@@ -42,6 +42,13 @@ int elem_type_of(const at::Tensor& t) {
   }
 }
 
+// A/B element type of the tcgen05 GEMM: 16-bit floats or 8-bit e4m3 / e5m2 (fp32 operands are refused, not reinterpreted)
+int gemm_input_dtype_of(const at::Tensor& t, const char* who) {
+  const int dt = gemm_dtype_of(t);
+  TORCH_CHECK(dt != tb::DT_FP32, who, ": A/B must be bf16, fp16, float8_e4m3fn or float8_e5m2, got ", t.scalar_type());
+  return dt;
+}
+
 cudaStream_t cur_stream() { return at::cuda::getCurrentCUDAStream().stream(); }
 
 // a: [G, M, K] (a_mn=false) or [G, K, M] (a_mn=true); b: [Gb, N, K] (b_mn=false) or [Gb, K, N] (b_mn=true);
@@ -68,9 +75,10 @@ void gemm_ex(const at::Tensor& a, const at::Tensor& b, at::Tensor& d, bool a_mn,
   TORCH_CHECK(d.size(0) == p.G && d.size(1) == p.M && d.size(2) == p.N, "tutel_b200.gemm: output shape mismatch");
   p.b_group_div = static_cast<int>(b_group_div > 0 ? b_group_div : 1);
   TORCH_CHECK(b.size(0) * p.b_group_div >= p.G, "tutel_b200.gemm: not enough B groups");
+  const int64_t gB = (p.G + p.b_group_div - 1) / p.b_group_div;   // B groups (and rows of bias / scale_b / colsum) in use
   p.a = a.data_ptr(); p.lda = a.stride(1); p.a_group_stride = a.stride(0); p.a_mn_major = a_mn;
   p.b = b.data_ptr(); p.ldb = b.stride(1); p.b_group_stride = b.stride(0); p.b_mn_major = b_mn;
-  p.in_dtype = gemm_dtype_of(a);
+  p.in_dtype = gemm_input_dtype_of(a, "tutel_b200.gemm");
   p.d = d.data_ptr(); p.ldd = d.stride(1); p.d_group_stride = d.stride(0);
   p.out_dtype = gemm_dtype_of(d);
   TORCH_CHECK(p.out_dtype <= tb::DT_FP32, "tutel_b200.gemm: output must be bf16/fp16/fp32");
@@ -80,12 +88,13 @@ void gemm_ex(const at::Tensor& a, const at::Tensor& b, at::Tensor& d, bool a_mn,
     TORCH_CHECK(bias->is_cuda() && bias->dim() == 2 && bias->stride(1) == 1 &&
                     (bias->scalar_type() == a.scalar_type() || (a.element_size() == 1 && bias->scalar_type() == d.scalar_type() && d.element_size() == 2)),
                 "tutel_b200.gemm: bias must be [Gb, N] of the input dtype (fp8 inputs: of the 16-bit output dtype)");
+    TORCH_CHECK(bias->size(1) == p.N && bias->size(0) >= gB, "tutel_b200.gemm: bias must be [>= ceil(G / b_group_div), N]");
     p.bias = bias->data_ptr();
     p.bias_group_stride = bias->stride(0);
   }
   if (aux.has_value() && aux->defined()) {
     TORCH_CHECK(aux->is_cuda() && aux->scalar_type() == d.scalar_type() && aux->dim() == 3 && aux->stride(2) == 1 &&
-                    aux->element_size() == 2,
+                    aux->element_size() == 2 && aux->size(0) == p.G && aux->size(1) == p.M && aux->size(2) == p.N,
                 "tutel_b200.gemm: aux must be a 16-bit [G, M, N] tensor of the output dtype");
     p.aux = aux->data_ptr();
     p.ld_aux = aux->stride(1);
@@ -103,13 +112,13 @@ void gemm_ex(const at::Tensor& a, const at::Tensor& b, at::Tensor& d, bool a_mn,
   }
   if (scale_b.has_value() && scale_b->defined()) {
     TORCH_CHECK(scale_b->is_cuda() && scale_b->scalar_type() == at::kFloat && scale_b->dim() == 2 && scale_b->stride(1) == 1 &&
-                scale_b->size(1) == p.N, "tutel_b200.gemm: scale_b must be float [Gb, N]");
+                scale_b->size(1) == p.N && scale_b->size(0) >= gB, "tutel_b200.gemm: scale_b must be float [>= ceil(G / b_group_div), N]");
     p.scale_b = scale_b->data_ptr<float>();
     p.scale_b_group_stride = scale_b->stride(0);
   }
   if (colsum.has_value() && colsum->defined()) {
     TORCH_CHECK(colsum->is_cuda() && colsum->scalar_type() == at::kFloat && colsum->dim() == 2 && colsum->stride(1) == 1 &&
-                colsum->size(1) == p.N, "tutel_b200.gemm: colsum must be float [Gb, N]");
+                colsum->size(1) == p.N && colsum->size(0) >= gB, "tutel_b200.gemm: colsum must be float [>= ceil(G / b_group_div), N]");
     p.colsum = colsum->data_ptr<float>();
     p.colsum_group_stride = colsum->stride(0);
   }
@@ -478,7 +487,7 @@ void gemm_glu(const at::Tensor& a, const at::Tensor& b, const c10::optional<at::
               const c10::optional<at::Tensor>& scale_a, const c10::optional<at::Tensor>& scale_b,
               const c10::optional<at::Tensor>& scale_b2, const c10::optional<at::Tensor>& row_counts,
               int64_t b_group_div, int64_t cta_group, int64_t wait_flags, int64_t wait_rows_per_flag,
-              int64_t wait_flags_per_group, int64_t wait_target, int64_t group_rot, int64_t group_mod) {
+              int64_t wait_flags_per_group, int64_t wait_target, int64_t group_rot, int64_t group_mod, int64_t max_ctas) {
   TORCH_CHECK(a.is_cuda() && b.is_cuda() && d.is_cuda() && a.dim() == 3 && b.dim() == 3 && d.dim() == 3);
   TORCH_CHECK(a.stride(2) == 1 && b.stride(2) == 1 && d.stride(2) == 1 && a.scalar_type() == b.scalar_type());
   const c10::cuda::CUDAGuard guard(a.device());
@@ -491,7 +500,9 @@ void gemm_glu(const at::Tensor& a, const at::Tensor& b, const c10::optional<at::
   TORCH_CHECK((b_mn ? b.size(1) : b.size(2)) == p.K, "tutel_b200.gemm_glu: K mismatch");
   p.b_group_div = static_cast<int>(b_group_div > 0 ? b_group_div : 1);
   TORCH_CHECK(b.size(0) * p.b_group_div >= p.G && d.size(0) == p.G && d.size(1) == p.M && d.size(2) == p.N && d.element_size() == 2);
+  const int64_t gB = (p.G + p.b_group_div - 1) / p.b_group_div;
   p.cta_group = static_cast<int>(cta_group);
+  p.max_ctas = static_cast<int>(max_ctas);
   p.wait_flags = reinterpret_cast<const uint32_t*>(wait_flags);
   p.wait_rows_per_flag = static_cast<int>(wait_rows_per_flag);
   p.wait_flags_per_group = static_cast<int>(wait_flags_per_group);
@@ -500,7 +511,7 @@ void gemm_glu(const at::Tensor& a, const at::Tensor& b, const c10::optional<at::
   p.group_mod = static_cast<int>(group_mod != 0 ? group_mod : 1);
   p.a = a.data_ptr(); p.lda = a.stride(1); p.a_group_stride = a.stride(0);
   p.b = b.data_ptr(); p.ldb = b.stride(1); p.b_group_stride = b.stride(0); p.b_mn_major = b_mn;
-  p.in_dtype = gemm_dtype_of(a);
+  p.in_dtype = gemm_input_dtype_of(a, "tutel_b200.gemm_glu");
   p.d = d.data_ptr(); p.ldd = d.stride(1); p.d_group_stride = d.stride(0);
   p.out_dtype = gemm_dtype_of(d);
   p.act = static_cast<int>(act);
@@ -526,16 +537,18 @@ void gemm_glu(const at::Tensor& a, const at::Tensor& b, const c10::optional<at::
     p.aux2 = aux2->data_ptr();
     p.d2 = d2->data_ptr();
   }
-  auto scale = [&](const c10::optional<at::Tensor>& t, int64_t cols, const float** ptr, long long* stride) {
+  auto scale = [&](const c10::optional<at::Tensor>& t, int64_t rows, int64_t cols, const float** ptr, long long* stride) {
     if (!t.has_value() || !t->defined()) return;
-    TORCH_CHECK(t->is_cuda() && t->scalar_type() == at::kFloat && t->dim() == 2 && t->stride(1) == 1 && t->size(1) == cols);
+    TORCH_CHECK(t->is_cuda() && t->scalar_type() == at::kFloat && t->dim() == 2 && t->stride(1) == 1 && t->size(0) >= rows &&
+                    t->size(1) == cols,
+                "tutel_b200.gemm_glu: scales must be float [G, M] (scale_a) or [>= ceil(G / b_group_div), N] (scale_b, scale_b2)");
     *ptr = t->data_ptr<float>();
     if (stride) *stride = t->stride(0);
   };
-  scale(scale_a, p.M, &p.scale_a, &p.scale_a_group_stride);
-  scale(scale_b, p.N, &p.scale_b, &p.scale_b_group_stride);
+  scale(scale_a, p.G, p.M, &p.scale_a, &p.scale_a_group_stride);
+  scale(scale_b, gB, p.N, &p.scale_b, &p.scale_b_group_stride);
   long long s2 = p.scale_b_group_stride;
-  scale(scale_b2, p.N, &p.scale_b2, &s2);
+  scale(scale_b2, gB, p.N, &p.scale_b2, &s2);
   TORCH_CHECK(s2 == p.scale_b_group_stride, "tutel_b200.gemm_glu: scale_b / scale_b2 stride mismatch");
   if (row_counts.has_value() && row_counts->defined()) {
     TORCH_CHECK(row_counts->is_cuda() && row_counts->scalar_type() == at::kInt && row_counts->numel() >= p.G);

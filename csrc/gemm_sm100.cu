@@ -809,7 +809,8 @@ gemm_sm100_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           if (XACT && args.d2 != nullptr && (args.epilogue == EPI_BIAS_GELU || args.epilogue == EPI_BIAS_SILU)) {
             // training: the backward pass needs the pre-activation (ReLU gets by with the sign of its output)
             uint8_t* d2_row = reinterpret_cast<uint8_t*>(args.d2) +
-                              (static_cast<long long>(tc.g) * args.d_group_stride + static_cast<long long>(m) * args.ldd) * 2;
+                              (static_cast<long long>(tc.g) * args.d_group_stride + static_cast<long long>(m) * args.ldd) *
+                                  (out16 ? 2 : 4);
             store_seg(&tmD2, d2_row, n, ncols, v);
           }
           if (args.epilogue == EPI_BIAS_RELU) {
@@ -1005,6 +1006,10 @@ cudaError_t gemm_sm100_launch(const GemmProblem& p, cudaStream_t stream, const c
   const char** why = why_out ? why_out : &why_local;
   *why = nullptr;
   if (p.M <= 0 || p.N <= 0 || p.K <= 0 || p.G <= 0) return cudaSuccess;
+  if (p.in_dtype != DT_BF16 && p.in_dtype != DT_FP16 && p.in_dtype != DT_E4M3 && p.in_dtype != DT_E5M2) {
+    *why = "A/B must be bf16, fp16, e4m3 or e5m2";
+    return cudaErrorInvalidValue;
+  }
   const int eb = (p.in_dtype == DT_E4M3 || p.in_dtype == DT_E5M2) ? 1 : 2;
   if (p.N % 8 != 0) { *why = "N must be a multiple of 8"; return cudaErrorInvalidValue; }
   const int ob = p.out_dtype == DT_FP32 ? 4 : 2;
@@ -1033,8 +1038,24 @@ cudaError_t gemm_sm100_launch(const GemmProblem& p, cudaStream_t stream, const c
   if (dual) bn = 256;
   if (cg == 0) cg = (p.M > 128) ? 2 : 1;
   if (cg == 2 && (sms & 1)) sms -= 1;
+  if (sms < cg) sms = cg;   // max_ctas = 1 with CTA pairs still runs one pair
 
   const int bm = 128 * cg;
+  // rotate_group() maps g into [0, G) only when |group_mod| divides G and 0 <= group_rot < |group_mod|.
+  const int rot_mod = p.group_mod < 0 ? -p.group_mod : p.group_mod;
+  if (p.group_rot < 0 || (rot_mod > 1 && (p.G % rot_mod != 0 || p.group_rot >= rot_mod))) {
+    *why = "group_mod must divide G and group_rot must lie in [0, |group_mod|)";
+    return cudaErrorInvalidValue;
+  }
+  // The producer remembers the arrival flags of the current group in a 64-bit mask.
+  if (p.wait_flags != nullptr) {
+    const int rows_per_flag = p.wait_rows_per_flag > 0 ? p.wait_rows_per_flag : bm;
+    const int flags = (p.M + rows_per_flag - 1) / rows_per_flag;
+    if (flags > 64 || flags > p.wait_flags_per_group) {
+      *why = "wait_flags: ceil(M / wait_rows_per_flag) must be at most 64 and at most wait_flags_per_group";
+      return cudaErrorInvalidValue;
+    }
+  }
   GemmArgs a{};
   a.M = p.M; a.N = p.N; a.K = p.K; a.G = p.G;
   a.b_group_div = p.b_group_div > 0 ? p.b_group_div : 1;

@@ -80,7 +80,8 @@ struct GemmProblem {
 
   // Optional dispatch fusion: before the A rows [m0, m0+BM) of group g are loaded, the TMA producer
   // acquires  wait_flags[g * wait_flags_per_group + m0 / wait_rows_per_flag] >= wait_target  (system scope);
-  // peers bump these counters after pushing token rows over NVLink.
+  // peers bump these counters after pushing token rows over NVLink.  ceil(M / wait_rows_per_flag) (rows per flag
+  // default to the tile height) must not exceed 64 nor wait_flags_per_group.
   const uint32_t* wait_flags = nullptr;
   int wait_rows_per_flag = 0, wait_flags_per_group = 0;
   uint32_t wait_target = 0;
@@ -88,17 +89,20 @@ struct GemmProblem {
   // usually in a peer's memory) is incremented with release.sys semantics.
   const unsigned long long* signal_ptr_table = nullptr;
   // Tile order: group g is visited as (g/mod)*mod + (g%mod + rot)%mod, so a rank can start with the segment whose
-  // rows it produced itself while the peers' rows are still in flight.
+  // rows it produced itself while the peers' rows are still in flight.  A negative mod visits the segment downwards.
+  // group_rot must be >= 0; when |mod| > 1, |mod| must divide G and group_rot must be < |mod|.
   int group_rot = 0, group_mod = 1;
 
   // Tuning: cta_group (1 or 2, 0 = auto), BN (128 or 256, 0 = auto)
   int cta_group = 0;
   int block_n = 0;
-  int max_ctas = 0;  // 0 = all SMs
+  int max_ctas = 0;  // 0 = all SMs; at least one CTA (one pair with cta_group 2) always runs
 };
 
 // Returns cudaSuccess or the launch error; throws nothing.  `why` (optional) receives a static message on
-// argument errors (misaligned strides etc.).
+// argument errors (misaligned strides, A/B not bf16 / fp16 / e4m3 / e5m2, group_rot / group_mod or wait-flag
+// counts out of range, etc.).  The sizes of the side tensors (bias, aux, scales, colsum) are not visible here: the
+// caller guarantees them (the torch bindings check them against the tensor shapes).
 cudaError_t gemm_sm100_launch(const GemmProblem& p, cudaStream_t stream, const char** why = nullptr);
 
 }  // namespace tb

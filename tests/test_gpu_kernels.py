@@ -12,58 +12,6 @@ def C():
     return backend.require_ext()
 
 
-def _gemm(C, a, b, d, a_mn, b_mn, epi=0, bias=None, aux=None, counts=None, cg=0, bn=0):
-    C.gemm(a, b, d, a_mn, b_mn, epi, bias, aux, counts, 1.0, 1, cg, bn, 0, 0, 0, 0, 0, 0, 0, 0, 1, None, None, None)
-
-
-@pytest.mark.parametrize('cg', [1, 2])
-@pytest.mark.parametrize('a_mn,b_mn', [(False, False), (False, True), (True, False), (True, True)])
-def test_tcgen05_gemm_all_layouts(C, cg, a_mn, b_mn):
-    torch.manual_seed(0)
-    G, M, N, K = 3, 328, 264, 200
-    a = (torch.randn(G, M, K, device='cuda') * 0.5).bfloat16()
-    b = (torch.randn(G, N, K, device='cuda') * 0.5).bfloat16()
-    a_op = a.transpose(1, 2).contiguous() if a_mn else a
-    b_op = b.transpose(1, 2).contiguous() if b_mn else b
-    d = torch.full((G, M, N), float('nan'), device='cuda', dtype=torch.bfloat16)
-    _gemm(C, a_op, b_op, d, a_mn, b_mn, cg=cg)
-    ref = torch.matmul(a.float(), b.float().transpose(1, 2))
-    assert torch.allclose(d.float(), ref, atol=0.08, rtol=2e-2)
-
-
-@pytest.mark.parametrize('dtype,out', [(torch.float16, torch.float16), (torch.bfloat16, torch.float32)])
-def test_tcgen05_gemm_dtypes_and_epilogues(C, dtype, out):
-    torch.manual_seed(1)
-    G, M, N, K = 2, 512, 520, 1096
-    a = (torch.randn(G, M, K, device='cuda') * 0.3).to(dtype)
-    b = (torch.randn(G, N, K, device='cuda') * 0.3).to(dtype)
-    bias = torch.randn(G, N, device='cuda').to(dtype)
-    d = torch.empty(G, M, N, device='cuda', dtype=out)
-    _gemm(C, a, b, d, False, False, epi=2, bias=bias)
-    ref = torch.relu(torch.matmul(a.float(), b.float().transpose(1, 2)) + bias.float().unsqueeze(1))
-    assert torch.allclose(d.float(), ref, atol=0.1, rtol=2e-2)
-    if out == torch.float32:
-        return          # the ReLU-gradient epilogue reads a 16-bit activation tensor of the output's dtype
-    aux = torch.randn(G, M, N, device='cuda').to(out)
-    _gemm(C, a, b, d, False, False, epi=5, aux=aux)
-    ref = torch.where(aux.float() > 0, torch.matmul(a.float(), b.float().transpose(1, 2)), torch.zeros((), device='cuda'))
-    assert torch.allclose(d.float(), ref, atol=0.1, rtol=2e-2)
-
-
-def test_tcgen05_gemm_row_counts_skip_tiles(C):
-    torch.manual_seed(2)
-    G, M, N, K = 4, 512, 256, 256
-    a = torch.randn(G, M, K, device='cuda').bfloat16()
-    b = torch.randn(G, N, K, device='cuda').bfloat16()
-    counts = torch.tensor([512, 0, 130, 257], device='cuda', dtype=torch.int32)
-    d = torch.full((G, M, N), 7.0, device='cuda', dtype=torch.bfloat16)
-    _gemm(C, a, b, d, False, False, counts=counts)
-    ref = torch.matmul(a.float(), b.float().transpose(1, 2))
-    for g, c in enumerate(counts.tolist()):
-        assert torch.allclose(d[g, :c].float(), ref[g, :c], atol=0.3, rtol=2e-2)
-        assert torch.all(d[g, (c + 255) // 256 * 256:] == 7.0)     # skipped tiles were never touched
-
-
 @pytest.mark.parametrize('S,E,k', [(8192, 8, 2), (5000, 130, 3), (33, 128, 1)])
 def test_routing_kernels_match_cpu(C, S, E, k):
     torch.manual_seed(S)
@@ -279,16 +227,6 @@ def test_glu_dual_b_gemm_forward_and_backward_epilogues(C, act, M, b_mn):
     (_act(act, gf) * uf).backward(dh)
     assert torch.allclose(dg.float(), gf.grad, atol=0.05, rtol=3e-2)
     assert torch.allclose(du.float(), uf.grad, atol=0.05, rtol=3e-2)
-
-
-def test_gemm_add_epilogue(C):
-    torch.manual_seed(4)
-    a = torch.randn(2, 300, 128, device='cuda').bfloat16()
-    b = torch.randn(2, 264, 128, device='cuda').bfloat16()
-    aux = torch.randn(2, 300, 264, device='cuda').bfloat16()
-    d = torch.empty_like(aux)
-    _gemm(C, a, b, d, False, False, epi=8, aux=aux)
-    assert torch.allclose(d.float(), a.float() @ b.float().transpose(1, 2) + aux.float(), atol=0.15, rtol=2e-2)
 
 
 @pytest.mark.parametrize('act', ['silu', 'relu'])

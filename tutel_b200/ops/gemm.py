@@ -405,7 +405,7 @@ def fused_relu_ffn_fp8(x, w1, b1, w2, b2, row_counts=None):
 def _glu_extra(kw):
     return (int(kw.get('b_group_div', 1)), int(kw.get('cta_group', 0)), int(kw.get('wait_flags', 0)),
             int(kw.get('wait_rows_per_flag', 0)), int(kw.get('wait_flags_per_group', 0)), int(kw.get('wait_target', 0)),
-            int(kw.get('group_rot', 0)), int(kw.get('group_mod', 1)))
+            int(kw.get('group_rot', 0)), int(kw.get('group_mod', 1)), int(kw.get('max_ctas', 0)))
 
 
 def glu_gemm(a, b, b2, *, b_mn, act, save_pre=False, scale_a=None, scale_b=None, scale_b2=None, row_counts=None,
